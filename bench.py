@@ -29,6 +29,7 @@ Multi-GPU (`--gpus N` under torchrun, one rank per GPU).  Default `--mode auto` 
   `--mode replica` / `--mode shard` run one form only (shard: `value` is the shard-mode QPS over the N-shard corpus).
 """
 import argparse
+import contextlib
 import json
 import os
 import subprocess
@@ -38,8 +39,11 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the index build runs with torch's deterministic algorithms (deterministic_build), which require a fixed cuBLAS
+# workspace configuration; cuBLAS reads it when its first handle is created, so it is set before torch is imported
+os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")
 
-BUILDER_VERSION = 3
+BUILDER_VERSION = 4   # 4: deterministic index build
 L2_BYTES = 126 * 1000 * 1000  # B200 L2 (B200_PROFILING.md)
 
 
@@ -57,6 +61,9 @@ def l2_policy_text(row_bytes_total):
 def log(*a):
     if int(os.environ.get("RANK", "0")) == 0:
         print("[bench]", *a, file=sys.stderr, flush=True)
+
+
+REFERENCE_DUMP_QUERIES = 256   # the least the reference arm's timed sample holds
 
 
 def parse_args():
@@ -96,7 +103,33 @@ def parse_args():
                     help="index holds uint8 PQ codes (BASELINE config 4 shape: --quantizer opq --raw-type int8 --dim 100 --pq-m 50)")
     ap.add_argument("--pq-m", type=int, default=50, help="number of PQ sub-vectors")
     ap.add_argument("--raw-type", default="float", choices=["float", "int8"], help="element type of raw vectors/queries")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result lists of the last timed step as DIR/ids.npy (float64) and DIR/dists.npy (float32); "
+                         "--impl reference writes its first %d queries (its per-step sample is sized by timing)" % REFERENCE_DUMP_QUERIES)
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(folder, ids, dists):
+    """What a caller of the timed path receives: ids [nq, k] as float64 (exact for int32 ids) and dists [nq, k] as
+    float32.  Above DUMP_LIMIT_BYTES a fixed, seeded sample of query rows is written, with its row numbers in rows.npy."""
+    import numpy as np
+    ids = np.asarray(ids).astype(np.float64)
+    dists = np.asarray(dists, dtype=np.float32)
+    row_bytes = ids.shape[1] * 8 + dists.shape[1] * 4 + 8
+    os.makedirs(folder, exist_ok=True)
+    if ids.shape[0] * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(ids.shape[0], DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        ids, dists = ids[rows], dists[rows]
+        np.save(os.path.join(folder, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(folder, "ids.npy"), ids)
+    np.save(os.path.join(folder, "dists.npy"), dists)
+    log("outputs of the last timed step written to %s" % folder)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -137,6 +170,20 @@ def gen_data(args, n, seed, device):
         # unit-norm queries from the caller
         x = x / x.norm(dim=1, keepdim=True).clamp_min(1e-30)
     return x.contiguous()
+
+
+@contextlib.contextmanager
+def deterministic_build():
+    """The index is an input of every timed step: build it with torch's deterministic kernels (index_add_ without float
+    atomics in the k-means) so that the same arguments give the same index, and the same outputs, on every run.  An op
+    without a deterministic implementation raises instead of building a different index."""
+    import torch
+    prev = torch.are_deterministic_algorithms_enabled()
+    torch.use_deterministic_algorithms(True)
+    try:
+        yield
+    finally:
+        torch.use_deterministic_algorithms(prev)
 
 
 def index_folder(args, shard):
@@ -180,11 +227,13 @@ def ensure_index(args, shard, device):
         return folder
     torch.backends.cuda.matmul.allow_tf32 = True
     x = gen_data(args, args.n, args.seed + 1000 * (shard + 1), device)
-    nodes, starts, graph = B.build_index(x, args.metric, seed=args.seed + shard, log=log, algo=args.algo.upper(),
-                                         tpt_above=args.tpt_above)
+    with deterministic_build():
+        nodes, starts, graph = B.build_index(x, args.metric, seed=args.seed + shard, log=log, algo=args.algo.upper(),
+                                             tpt_above=args.tpt_above)
     if args.quantizer != "none":
-        cb, rot = B.train_quantizer_gpu(x, args.pq_m, opq=(args.quantizer == "opq"), seed=args.seed)
-        codes = B.encode_gpu(x, cb, rot)
+        with deterministic_build():
+            cb, rot = B.train_quantizer_gpu(x, args.pq_m, opq=(args.quantizer == "opq"), seed=args.seed)
+            codes = B.encode_gpu(x, cb, rot)
         blob = B.quantizer_blob(cb, rot, 0 if args.raw_type == "int8" else 3)
         B.save_index_folder(folder, codes.cpu().numpy(), graph, nodes, starts, args.metric, quantizer=blob)
     elif args.raw_type == "int8":   # unquantized int8 rows (DistanceUtils int8 variants), e.g. SPACEV / PerfTest.cpp shape
@@ -221,8 +270,9 @@ def build_in_memory(args, shard, device):
     t0 = time.time()
     torch.backends.cuda.matmul.allow_tf32 = True
     x = gen_data(args, args.n, args.seed + 1000 * (shard + 1), device)
-    nodes, starts, graph = B.build_index(x, args.metric, seed=args.seed + shard, log=log, algo=args.algo.upper(),
-                                         tpt_above=args.tpt_above)
+    with deterministic_build():
+        nodes, starts, graph = B.build_index(x, args.metric, seed=args.seed + shard, log=log, algo=args.algo.upper(),
+                                             tpt_above=args.tpt_above)
     torch.backends.cuda.matmul.allow_tf32 = False
     files = _InMemoryIndex(x.cpu().numpy(), graph, nodes, starts, args.metric)
     del x
@@ -410,7 +460,7 @@ def main():
             idx.set_param("MaxCheck", args.maxcheck)
             kind = "reference"
             for s in range(args.warmup + args.steps):
-                _, _, sec = (idx.search_each if quantized else idx.search)(q[:sample], args.k, threads=threads)
+                ids, dists, sec = (idx.search_each if quantized else idx.search)(q[:sample], args.k, threads=threads)
                 if s >= args.warmup:
                     secs.append(sec)
         else:
@@ -419,9 +469,11 @@ def main():
             o.max_check = args.maxcheck
             for s in range(args.warmup + args.steps):
                 t = time.time()
-                o.search(q[:sample], args.k, threads=threads, want_stats=False)
+                ids, dists, _ = o.search(q[:sample], args.k, threads=threads, want_stats=False)
                 if s >= args.warmup:
                     secs.append(time.time() - t)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ids[:REFERENCE_DUMP_QUERIES], dists[:REFERENCE_DUMP_QUERIES])
         total = sum(secs)
         qps = sample * len(secs) / total
         line = {"impl": "reference", "metric": "queries_per_second", "value": qps, "unit": "queries/s",
@@ -622,6 +674,8 @@ def main_leg(args, rank, local_rank, world, dev, dist, quantized, config, mode):
     sync_all()
     tm1 = time.time()
     launches = capi.launch_count() - launches0
+    if args.dump_outputs:
+        last_ids, last_dists = d_ids.cpu().numpy(), d_dists.cpu().numpy()
     ms_total = ev0.elapsed_time(ev1)
     if world > 1:
         t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
@@ -695,6 +749,8 @@ def main_leg(args, rank, local_rank, world, dev, dist, quantized, config, mode):
     if rank != 0:
         idx.close()
         return None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_ids, last_dists)
 
     # ---- roofline of the dominant (only) kernel of a step ----
     peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
@@ -895,6 +951,8 @@ def shard_leg(args, rank, local_rank, world, dev, dist, config):
     sync_all()
     tm1 = time.time()
     launches = capi.launch_count() - launches0
+    if rank == 0 and args.dump_outputs and args.mode == "shard":
+        dump_outputs(args.dump_outputs, m_ids.cpu().numpy(), m_d.cpu().numpy())
     ms_total = ev0.elapsed_time(ev1)
     exch_ms = sum(marks[2 * i].elapsed_time(marks[2 * i + 1]) for i in range(len(marks) // 2)) / max(1, len(marks) // 2)
     t = torch.tensor([ms_total, exch_ms], dtype=torch.float64, device=dev)

@@ -5,7 +5,7 @@ types (BasicResult with Meta, QueryResult, ResultIterator, WorkSpace) next to th
 SearchIndex(batch) with and without metadata, the AnnIndex::BatchSearch / Search patterns (Wrappers/src/CoreInterface.cpp
 :206-238), p_searchDeleted, SearchIndexWithFilter, RefineSearchIndex, GetIterator (the reference's ResultIterator class
 on top of the overridden virtuals), SPANN's head-index pattern (SPANNIndex.cpp:259-285) and a DeleteIndex + re-sync.
-The binary is built where /root/reference exists (build()); the GPU box runs the prebuilt one."""
+The binary is built into oracle/_ref by build() where the reference sources exist."""
 import os
 import subprocess
 import tempfile
@@ -17,7 +17,7 @@ from conftest import data_folder
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "tests", "cpp", "vector_index_dropin")
+EXE = os.path.join(ROOT, "oracle", "_ref", "vector_index_dropin")
 
 
 @pytest.mark.parametrize("name,k,mc", [("bkt_l2_10k_128", 10, 1024), ("bkt_cos_3k_768", 10, 8192),
@@ -29,7 +29,7 @@ def test_vector_index_subclass_matches_the_reference(name, k, mc):
     import __graft_entry__
     __graft_entry__.build_dropin_test()
     if not os.path.exists(EXE):
-        pytest.skip("tests/cpp/vector_index_dropin was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/vector_index_dropin was not built (needs the reference sources at build time)")
     folder = data_folder(name)
     q = np.load(os.path.join(folder, "queries.npy"))[:96]
     with tempfile.TemporaryDirectory() as tmp:

@@ -14,14 +14,14 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "tests", "cpp", "spann_head_dropin")
+EXE = os.path.join(ROOT, "oracle", "_ref", "spann_head_dropin")
 
 
 def test_spann_head_search_on_the_device():
     import __graft_entry__
     __graft_entry__.build_dropin_test()
     if not os.path.exists(EXE):
-        pytest.skip("tests/cpp/spann_head_dropin was not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/spann_head_dropin was not built (needs the reference sources at build time)")
     with tempfile.TemporaryDirectory() as tmp:
         r = subprocess.run([EXE, tmp], capture_output=True, text=True, timeout=900, cwd=tmp)
     lines = [l for l in r.stdout.splitlines() if l.startswith(("PASS", "FAIL"))]

@@ -237,26 +237,80 @@ def test_oracle_iterator_matches_golden_reference_outputs(oracle_lib, name):
 
 
 # ---------------------------------------------------------------------------------------------
-# the reference itself
+# the reference's outputs on seeded inputs, stored in tests/golden/pin/ (tests/golden/make_golden_pin.py)
 # ---------------------------------------------------------------------------------------------
-@needs_ref
+ISA_WIDTHS = [(512, 16), (256, 8), (128, 4), (0, 1)]
+F32_DIMS = [1, 2, 3, 4, 5, 7, 8, 9, 12, 15, 16, 17, 20, 24, 28, 31, 32, 33, 48, 63, 64, 100, 127, 128, 131, 200,
+            256, 384, 768, 960, 1000, 1024]
+F32_PAIRS = 300
+F32_PAIRS_KEPT = 48          # pairs per dimension whose reference distances are stored
+INT_CASES = [(reflib.VT_INT8, np.int8, -127, 128), (reflib.VT_UINT8, np.uint8, 0, 256),
+             (reflib.VT_INT16, np.int16, -32768, 32768), (reflib.VT_INT16, np.int16, -3000, 3000)]
+INT_DIMS = [1, 3, 4, 5, 15, 16, 17, 31, 32, 33, 47, 48, 63, 64, 65, 79, 80, 95, 96, 100, 127, 128, 131, 192, 200, 256, 258]
+INT_PAIRS = 25
+QUANTIZER_CASES = [(False, reflib.VT_FLOAT), (True, reflib.VT_FLOAT), (True, reflib.VT_INT8)]
+QUANT_ROWS_KEPT, QUANT_RECON_KEPT = 1000, 128
+
+
+def pin_golden(name):
+    return np.load(os.path.join(GOLDEN, "pin", name + ".npz"))
+
+
+def f32_distance_inputs():
+    """(dim, a [F32_PAIRS, dim], b [F32_PAIRS, dim]) per dimension of F32_DIMS."""
+    rng = np.random.default_rng(7)
+    for dim in F32_DIMS:
+        a = rng.standard_normal((F32_PAIRS, dim), dtype=np.float32)
+        b = rng.standard_normal((F32_PAIRS, dim), dtype=np.float32)
+        yield dim, a, b
+
+
+def int_distance_inputs(dt, lo, hi):
+    """(metric, dim, a, b) in the order the pairs are drawn."""
+    rng = np.random.default_rng(9)
+    for metric in (0, 1):
+        for dim in INT_DIMS:
+            for _ in range(INT_PAIRS):
+                a = rng.integers(lo, hi, dim).astype(dt)
+                b = rng.integers(lo, hi, dim).astype(dt)
+                yield metric, dim, a, b
+
+
+def int_case_key(vt, lo, hi):
+    return "vt%d_%d_%d" % (vt, lo, hi)
+
+
+def quantizer_rows(rtype):
+    """Low-rank raw rows (reflib.gen_lowrank's model) drawn without BLAS: the rank-6 product is summed term by term in
+    float32, so the rows are the same bits on every CPU."""
+    rng = np.random.default_rng(51)
+    a = rng.standard_normal((6, 24), dtype=np.float32) / np.float32(np.sqrt(6))
+    z = rng.standard_normal((3000, 6), dtype=np.float32)
+    x = np.zeros((3000, 24), np.float32)
+    for j in range(6):
+        x += z[:, j:j + 1] * a[j]
+    x += np.float32(0.1) * rng.standard_normal((3000, 24), dtype=np.float32)
+    return x if rtype == reflib.VT_FLOAT else np.clip(np.round(x * 32), -127, 127).astype(np.int8)
+
+
+def quantizer_case_key(opq, rtype):
+    return "%s_vt%d" % ("opq" if opq else "pq", rtype)
+
+
 @pytest.mark.parametrize("metric", [0, 1])
 def test_distance_bit_exact_vs_reference_all_trees(oracle_lib, metric):
-    rng = np.random.default_rng(7)
-    R = reflib.ref()
-    for dim in [1, 2, 3, 4, 5, 7, 8, 9, 12, 15, 16, 17, 20, 24, 28, 31, 32, 33, 48, 63, 64, 100, 127, 128, 131, 200,
-                256, 384, 768, 960, 1000, 1024]:
-        n = 300
-        a = rng.standard_normal((n, dim), dtype=np.float32)
-        b = rng.standard_normal((n, dim), dtype=np.float32)
-        for isa, width in [(512, 16), (256, 8), (128, 4), (0, 1)]:
-            out_r = np.empty(n, np.float32)
-            out_o = np.empty(n, np.float32)
-            R.ref_distance_f32_many(isa, metric, a.ctypes.data, b.ctypes.data, dim, n, out_r.ctypes.data)
-            oracle_lib.ora_distance_f32_many(metric, width, a.ctypes.data, b.ctypes.data, dim, n, out_o.ctypes.data)
-            assert np.array_equal(out_r.view(np.int32), out_o.view(np.int32)), (dim, isa)
+    """The reference's float DistanceUtils variants (AVX-512, AVX, SSE, scalar) against the oracle's SIMD trees."""
+    ref = pin_golden("distance_f32")["dists"][metric]                     # [dim, isa, pair]
+    for i, (dim, a, b) in enumerate(f32_distance_inputs()):
+        for j, (isa, width) in enumerate(ISA_WIDTHS):
+            out_o = np.empty(F32_PAIRS, np.float32)
+            oracle_lib.ora_distance_f32_many(metric, width, a.ctypes.data, b.ctypes.data, dim, F32_PAIRS, out_o.ctypes.data)
+            assert np.array_equal(out_o[:F32_PAIRS_KEPT].view(np.int32), ref[i, j].view(np.int32)), (dim, isa)
 
 
+# ---------------------------------------------------------------------------------------------
+# the reference itself, on the index folders it built (tests/make_test_data.py)
+# ---------------------------------------------------------------------------------------------
 @needs_ref
 @pytest.mark.parametrize("name", ["algo_line_bkt", "bkt_l2_20k_32", "bkt_cos_10k_128", "bkt_l2_5k_100",
                                   "bkt_l2_3k_30", "bkt_l2_dups", "kdt_l2_10k_64", "bkt2_l2_6k_32", "kdt2_l2_6k_32"])
@@ -299,24 +353,22 @@ def test_counters_match_reference_workspace(oracle_lib):
 # ---------------------------------------------------------------------------------------------
 # PQ / OPQ quantized indexes (SURVEY.md 8a row A10)
 # ---------------------------------------------------------------------------------------------
-@needs_ref
-@pytest.mark.parametrize("opq,rtype", [(False, reflib.VT_FLOAT), (True, reflib.VT_FLOAT), (True, reflib.VT_INT8)])
+@pytest.mark.parametrize("opq,rtype", QUANTIZER_CASES)
 def test_quantizer_bit_exact_vs_reference(oracle_lib, tmp_path, opq, rtype):
-    x = reflib.gen_lowrank(3000, 24, 6, 51)
-    xs = x if rtype == reflib.VT_FLOAT else np.clip(np.round(x * 32), -127, 127).astype(np.int8)
-    qz = reflib.train_quantizer(xs.astype(np.float32), m=6, ks=256, opq=opq, rtype=rtype, iters=2)
+    """PQ / OPQ QuantizeVector, SDC L2, ReconstructVector and re-quantisation of the reference, on the stored quantizer."""
+    g = pin_golden("quantizer_" + quantizer_case_key(opq, rtype))
+    xs = quantizer_rows(rtype)
     path = str(tmp_path / "q.bin")
-    qz.write(path)
-    rq = reflib.RefQuantizer(path)
+    g["quantizer_blob"].tofile(path)
     oq = reflib.OracleQuantizer(reflib.Quantizer.read(path))
-    cr, co = rq.encode(xs), oq.encode(xs)
-    assert np.array_equal(cr, co)                       # QuantizeVector (incl. the OPQ rotation)
-    dr = np.array([rq.l2(cr[i], cr[i + 1]) for i in range(500)], np.float32)
+    co = oq.encode(xs)
+    assert np.array_equal(co[:QUANT_ROWS_KEPT], g["codes"])                   # QuantizeVector (incl. the OPQ rotation)
     do = np.array([oq.l2(co[i], co[i + 1]) for i in range(500)], np.float32)
-    assert np.array_equal(dr.view(np.int32), do.view(np.int32))   # SDC table sum
-    rr, ro = rq.reconstruct(cr, xs.dtype), oq.reconstruct(co, xs.dtype)
-    assert np.array_equal(rr.view(np.uint8), ro.view(np.uint8))   # ReconstructVector (incl. the OPQ back-rotation + cast)
-    assert np.array_equal(rq.encode(rr), oq.encode(ro))           # ... and what RefineNode makes of it (SetTarget)
+    assert np.array_equal(do.view(np.int32), g["sdc_l2"].view(np.int32))     # SDC table sum
+    ro = oq.reconstruct(co, xs.dtype)
+    # ReconstructVector (incl. the OPQ back-rotation + cast) and what RefineNode makes of it (SetTarget)
+    assert np.array_equal(ro[:QUANT_RECON_KEPT].view(np.uint8), g["reconstructed"].view(np.uint8))
+    assert np.array_equal(oq.encode(ro)[:QUANT_ROWS_KEPT], g["recoded"])
 
 
 @needs_ref
@@ -340,24 +392,17 @@ def test_quantized_search_bit_exact_vs_reference(oracle_lib, name):
 # ---------------------------------------------------------------------------------------------
 # int8 / uint8 element types (DistanceUtils.cpp:305-558, :684-874)
 # ---------------------------------------------------------------------------------------------
-@needs_ref
-@pytest.mark.parametrize("vt,dt,lo,hi", [(reflib.VT_INT8, np.int8, -127, 128), (reflib.VT_UINT8, np.uint8, 0, 256),
-                                         (reflib.VT_INT16, np.int16, -32768, 32768),
-                                         (reflib.VT_INT16, np.int16, -3000, 3000)])
+@pytest.mark.parametrize("vt,dt,lo,hi", INT_CASES)
 def test_integer_distance_bit_exact_vs_reference(oracle_lib, vt, dt, lo, hi):
-    rng = np.random.default_rng(9)
-    width = {512: 16, 256: 8, 128: 4, 0: 1}[reflib.ref().ref_isa()]
+    """The reference's integer DistanceUtils, run through its own cpuid dispatch; `width` is the SIMD tree it picked."""
+    g = pin_golden("distance_int")
+    width = int(g["width"])
     if vt == reflib.VT_INT16 and width != 16:
         pytest.skip("the int16 restatement covers the AVX-512 variants only")
-    for metric in (0, 1):
-        for dim in [1, 3, 4, 5, 15, 16, 17, 31, 32, 33, 47, 48, 63, 64, 65, 79, 80, 95, 96, 100, 127, 128, 131, 192,
-                    200, 256, 258]:
-            for _ in range(25):
-                a = rng.integers(lo, hi, dim).astype(dt)
-                b = rng.integers(lo, hi, dim).astype(dt)
-                r = np.float32(reflib.ref().ref_distance(metric, vt, a.ctypes.data, b.ctypes.data, dim))
-                o = np.float32(oracle_lib.ora_distance(metric, vt, width, a.ctypes.data, b.ctypes.data, dim))
-                assert r.view(np.int32) == o.view(np.int32), (vt, metric, dim)
+    ref = g[int_case_key(vt, lo, hi)]
+    for i, (metric, dim, a, b) in enumerate(int_distance_inputs(dt, lo, hi)):
+        o = np.float32(oracle_lib.ora_distance(metric, vt, width, a.ctypes.data, b.ctypes.data, dim))
+        assert ref[i].view(np.int32) == o.view(np.int32), (vt, metric, dim)
 
 
 @needs_ref
